@@ -10,6 +10,8 @@ outside the hot path, SURVEY.md §8d).  Metric: megapixels of INPUT per second.
 
   python bench.py [--gpus N --steps K --warmup W]       our engine (one rank per GPU)
   python bench.py --impl reference [...]                 the reference's CPU path
+  python bench.py --dump-outputs DIR [...]               also write what the last timed step
+                                                         computed to DIR/*.npy (rank 0)
 
 Prints ONE JSON line on rank 0 (contract in the task statement):
   value    : K steps with inputs resident in HBM (device-timed, max over ranks)
@@ -74,6 +76,33 @@ def algorithmic_bytes(imgs, items, params, counts):
     """Per-launch algorithmic traffic of each kernel (SURVEY.md §8d model; tools/bench_configs.py)."""
     from tools.bench_configs import algorithmic_bytes as ab
     return ab([im.shape[:2] for im in imgs], items, params, counts, params.multiband)
+
+
+DUMP_BYTES = 64_000_000
+MOSAIC_SAMPLE_PIXELS = 1 << 20
+
+
+def dump_outputs(out_dir, fs, match_total, mosaic):
+    """What one step of the timed path hands its caller, so that two builds can be compared output
+    for output on the same seeded workload: every image's keypoint coordinates (f64) and descriptors
+    (f32), concatenated in image order, the per-image feature counts, the match total and the mosaic.
+    The mosaic (7500x1112x3 f32, 100 MB) is written as a fixed, seeded sample of its pixels
+    (mosaic_sample_index: the flat pixel indices, row-major) to keep the dump under DUMP_BYTES."""
+    feats = [fs.download(i) for i in range(fs.n_images)]
+    pixels = mosaic.reshape(-1, 3)
+    pick = np.arange(len(pixels))
+    if len(pixels) > MOSAIC_SAMPLE_PIXELS:
+        pick = np.sort(np.random.default_rng(0).choice(len(pixels), MOSAIC_SAMPLE_PIXELS, replace=False))
+    arrays = {"keypoints": np.concatenate([c for c, _ in feats]), "descriptors": np.concatenate([d for _, d in feats]),
+              "feature_counts": np.array([len(c) for c, _ in feats], np.float64),
+              "match_total": np.array([match_total], np.float64),
+              "mosaic_sample": pixels[pick], "mosaic_sample_index": pick.astype(np.float64)}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"bench.py: outputs of one step take {total} bytes, more than the dump's {DUMP_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def config_dict(imgs, pairs, bands, world, extra=None):
@@ -252,6 +281,8 @@ def main():
                     help="extra BASELINE.json configs measured in the same run at N=1 (comma list of 2mb,3,4,5; "
                          "'all'; 'none').  N>1 adds the sharded config-3 leg instead.")
     ap.add_argument("--sweep-sizes", default="10000,50000,100000,500000")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     # The contract is ONE JSON line on stdout.  Libraries chat on fd 1 (NCCL's version banner, the
     # reference's timers): keep a private handle to the real stdout for the line and point fd 1 at
@@ -264,8 +295,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
-        if args.steps > 5:
-            args.steps = 5          # bounded: each step is the full CPU workload (seconds)
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the CUDA arm's outputs; the reference arm has none to write")
         args.warmup = min(args.warmup, 1)
         run_reference(args, rank, world)
         return
@@ -315,9 +346,11 @@ def main():
             raise SystemExit("bench.py: degenerate workload (no features / matches)")
 
         # ---- value: inputs resident in HBM
-        def step_device():
-            f, _ = st.run_device(pairs, items, geom, args.bands, want_matches=False)
-            f.free()
+        def step_device(keep=False):
+            f, total = st.run_device(pairs, items, geom, args.bands, want_matches=False)
+            if not keep:
+                f.free()
+            return f, total
 
         import gc
         gc.collect()
@@ -334,13 +367,19 @@ def main():
         l0 = eng.launch_count()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        for _ in range(args.steps):
-            step_device()
+        for i in range(args.steps):
+            last = step_device(keep=bool(args.dump_outputs) and i == args.steps - 1)
         e1.record(stream)
         torch.cuda.synchronize()
         barrier()
         launches = eng.launch_count() - l0
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs:
+            if rank == 0:
+                mosaic = np.empty((out_h, out_w, 3), np.float32)
+                eng.dev_download(mosaic, st._d_out)          # the e2e legs below reuse the stitcher's canvas
+                dump_outputs(args.dump_outputs, last[0], last[1], mosaic)
+            last[0].free()
         exact_rows = eng.match_last_exact_rows()
         ms = e0.elapsed_time(e1)
         t_dev = torch.tensor([ms], device="cuda")

@@ -23,16 +23,6 @@ def orc():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The reference's own translation units (oracle/_ref); absent only if the
-    prebuilt .so did not travel."""
-    from tests.checker import get_checker, have
-    if not have("ref"):
-        pytest.skip("oracle/_ref/libopenpano_ref.so not built (needs /root/reference)")
-    return get_checker("ref")
-
-
-@pytest.fixture(scope="session")
 def engine():
     from openpano_b200.capi import Engine
     eng = Engine(0)

@@ -61,6 +61,62 @@ def ba(ref):
     print("ba:", len(pairs), "pairs,", len(pts), "matches")
 
 
+_RATIO_SCRIPT = """
+import json, sys
+sys.path.insert(0, {root!r})
+from tests import ref_cases as rc
+from tests.checker import get_checker
+print(json.dumps(rc.summary(rc.match_other_ratios(get_checker('ref'), {ratio}))))
+"""
+
+
+def ref_cases(ref):
+    """The reference's outputs of every case of tests/test_oracle_vs_ref.py (tests/ref_cases.py)."""
+    import json
+    import subprocess
+    from tests import ref_cases as rc
+    from tests.ba_util import ba_case
+    g = {}
+
+    def put(fn, *args):
+        g[rc.key(fn.__name__, *args)] = rc.summary(fn(ref, *args))
+
+    for args in rc.SIFT_SHAPES:
+        put(rc.sift_every_stage, *args)
+    put(rc.sift_other_params)
+    for args in rc.WIDE_WINDOWS:
+        put(rc.sift_wide_windows, *args)
+    put(rc.sift_flat_image)
+    put(rc.match_ragged_and_ties)
+    for args in rc.WARP_SHAPES:
+        put(rc.cyl_warp, *args)
+    put(rc.cyl_warp_other_focal)
+    for projection in rc.PROJECTIONS:
+        for bands in rc.PROJECTION_BANDS:
+            put(rc.blend_projections, projection, bands)
+    for args in rc.LAZY_ORDERED:
+        put(rc.blend_scaled_resolution, *args)
+    put(rc.imgio_read_write)
+    put(rc.imgio_crop)
+    for args in rc.RANSAC_CASES:
+        put(rc.ransac_scoring, *args)
+    for ratio, _, _ in rc.RATIOS:      # the reference freezes the ratio at its first match: one process each
+        out = subprocess.run([sys.executable, "-c", _RATIO_SCRIPT.format(root=str(ROOT), ratio=ratio)],
+                             capture_output=True, text=True, check=True)
+        g[rc.key("match_other_ratios", ratio)] = json.loads(out.stdout.strip().splitlines()[-1])
+    mats = {}
+    for args in rc.BA_CASES:
+        n_cam, per_pair, seed, extra = args
+        cams, pairs, pts = ba_case(n_cam, per_pair, seed, extra_pairs=extra)
+        k = rc.key("ba_jacobian", *args)
+        mats[k] = ref.ba_pair_mats(cams, pairs)
+        rows, jtj = ref.ba_jacobian_ref(cams, pairs, pts)
+        g[k] = rc.summary({"input": pts, "rows": rows, "jtj": jtj})
+    np.savez_compressed(OUT / rc.BA_MATS, **mats)
+    rc.GOLDEN_JSON.write_text(json.dumps(g, indent=1, sort_keys=True) + "\n")
+    print("ref_cases:", len(g), "cases")
+
+
 def main():
     ref = get_checker("ref")
     assert ref.num_threads() == 1
@@ -70,8 +126,12 @@ def main():
     if sys.argv[1:] == ["ba"]:
         ba(ref)
         return
+    if sys.argv[1:] == ["ref_cases"]:
+        ref_cases(ref)
+        return
     imgio(ref)
     ba(ref)
+    ref_cases(ref)
 
     # ---- SIFT chain on one 240x180 view
     img = synth.make_canvas(180, 240, 101)
